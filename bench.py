@@ -1,6 +1,6 @@
 """bench.py -- Mpaths/s of the ReSTIR PT frame (1 spp, 1920x1080, Cornell Box) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step is one frame of the reference's frame graph for the emissive Cornell Box, steady state (temporal and
@@ -18,6 +18,9 @@ temporal + spatial path reuse) -> compositing + firefly filter -> TAA. Nothing i
   c1_alias_table  config C1: alias-table build, device (zr_alias_table_build) next to the CPU reference-equivalent
   --impl reference   the same CPU path with every host core (SURVEY 8d: the only CPU arm the reference's math has); this arm
                   does not map libzetaray_b200.so (ZETARAY_B200_STRUCTS_ONLY)
+  --dump-outputs DIR  after the timed frames, the image the last of them produced (what Renderer.GetOutput() hands the
+                  caller: RGBA16F, 1080 x 1920 x 4) is written as DIR/image.npy in float32 (32 MB). The inputs depend only on the
+                  arguments, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -32,6 +35,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the source tree (it may be read-only)
 
 W, H = 1920, 1080
 METRIC = "Mpaths/s (1spp ReSTIR PT, 1080p)"
@@ -181,9 +185,8 @@ def run_reference(args):
     cores = os.cpu_count() or 1
     sw, sh = 960, 540
     # one renderer, `warmup` frames to reach steady state (temporal + spatial reuse on), then the timed frames
-    nsteps = max(1, min(args.steps, 60))
-    mp, spf = cpu_frames(sw, sh, nsteps, cores, warm=max(3, args.warmup))
-    per = [(mp, spf)] * nsteps
+    mp, spf = cpu_frames(sw, sh, args.steps, cores, warm=max(3, args.warmup))
+    per = [(mp, spf)] * args.steps
     sample = "%d steady-state frame(s) at %dx%d (1/4 of the 1080p pixels), %d threads" % (len(per), sw, sh, cores)
     line = {
         "impl": "reference", "metric": METRIC, "value": mp, "unit": "Mpaths/s", "n_gpus": args.gpus, "steps": len(per),
@@ -205,8 +208,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--single-stream", action="store_true", help="record DirectLighting on the main stream instead of a second one")
     ap.add_argument("--schedule-by-cost", action="store_true", help="N > 1: launch the lighting kernels' blocks most-expensive-tile-first (measured cost map)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the image of the last timed frame to DIR/image.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to the device path, not to --impl reference")
         run_reference(args)
         return
     args.warmup = max(args.warmup, 3)
@@ -319,6 +327,10 @@ def main():
     stop.set()
     ms = e0.elapsed_time(e1)
     launches = lib.zr_kernel_launch_count() - launches0
+    dumped = None
+    if args.dump_outputs and rank == 0:     # outside the timed region, before any later frame overwrites the image
+        from zetaray_b200.passes import download_image
+        dumped = {"image": download_image(output_image(), np.float16, 4).reshape(H, W, 4).astype(np.float32)}
     t = torch.tensor([ms], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -497,6 +509,10 @@ def main():
             "roofline": roofline, "kernels": kernels, "cpu_baseline": cpu, "c1_alias_table": c1, "with_svgf": with_svgf,
         }
         print(json.dumps(line))
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     if world > 1:
         dist.destroy_process_group()
 

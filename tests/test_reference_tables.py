@@ -1,13 +1,15 @@
 """The constant tables that define the reference's result are the reference's own bytes (VERDICT r1, item 1a):
 the 512-point disk of ReSTIR PT's spatial search (IndirectLighting/ReSTIR_PT/SampleSet.hlsli:8-523), the 32-point set
 of ReSTIR DI's spatial pass (DirectLighting/Emissive/Resampling.hlsli:352-386) and the directional-albedo volume
-Assets/LUT/rho.dds. With the reference tree present the committed assets are compared byte for byte with a fresh
-extraction; without it (GPU box) their SHA-256 is compared with the values recorded here at extraction time."""
+Assets/LUT/rho.dds. The committed assets are compared byte for byte with an extraction from the reference tree, frozen in
+tests/golden/reference_tables.npz by `reference_outputs`, and their SHA-256 with the values recorded here at extraction time."""
 import hashlib
 import os
 import sys
 import numpy as np
 import pytest
+
+from tests.golden_pins import Golden, pin
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ASSETS = os.path.join(ROOT, "zetaray_b200", "assets")
@@ -23,13 +25,17 @@ def test_asset_hash(name):
     assert hashlib.sha256(open(os.path.join(ASSETS, name), "rb").read()).hexdigest() == SHA256[name]
 
 
-def test_assets_are_the_reference_bytes():
-    if not os.path.isdir("/root/reference/Source"):
-        pytest.skip("reference tree not available on this machine")
+def reference_outputs():
+    """The three tables as tools/extract_reference_tables.py reads them from the reference tree."""
     sys.path.insert(0, os.path.join(ROOT, "tools"))
     import extract_reference_tables as ert
-    for name, arr in ert.tables().items():
-        assert open(os.path.join(ASSETS, name), "rb").read() == arr.tobytes(), name
+    return {name: pin(arr) for name, arr in ert.tables().items()}
+
+
+def test_assets_are_the_reference_bytes():
+    ref = Golden("reference_tables.npz")
+    for name in sorted(SHA256):
+        ref.check(name, np.fromfile(os.path.join(ASSETS, name), dtype=np.uint8).reshape(-1, ref[name + ".rows"].shape[1]))
 
 
 def test_table_shapes_and_ranges():

@@ -8,7 +8,7 @@ indices of both spatial passes and every dielectric-reflectance lookup differ fr
 
 half2 literals are float32 literals narrowed to binary16 (round to nearest even); the .bin files hold them widened back to
 float32, the form the kernels and the oracle consume. `--check` compares the committed assets with the reference tree
-instead of writing (tests/test_reference_tables.py does the same when /root/reference is present)."""
+instead of writing (tests/test_reference_tables.py compares them with an extraction frozen in tests/golden/reference_tables.npz)."""
 import os
 import re
 import struct
